@@ -4,6 +4,7 @@ steps, CFG 7.5, guidance active on the early steps), one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
     python bench.py --impl reference [...]                       # the reference's algorithm on the host cores (oracle port)
+    python bench.py [...] --dump-outputs DIR                     # also write the last timed image's latents to DIR
 
 A "step" is one guided image (50 denoising steps of the per-step guidance path + the UNet passes that drive it).
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
@@ -246,6 +247,14 @@ def _sha(t):
     return hashlib.sha1(t.detach().to(torch.float16).cpu().contiguous().numpy().tobytes()).hexdigest()[:16]
 
 
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs`: every array as `out_dir/<name>.npy` in float32.  The inputs are fixed by the seeds above, so two
+    builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def build_pipeline(args, dev):
     from guided_attention_b200 import run as R
     from guided_attention_b200.pipeline_guided_attention import GuidedAttention
@@ -333,6 +342,7 @@ def run_ours(args):
     pipe._count_pass("cfg", 0)
     before = dict(pipe.pass_counts)
     ms_value, value_res = timed(lambda i: image(seed_of(i), embeds_dev, dev_lat[i]), args.steps)
+    last_out = value_res[-1].detach().cpu() if args.dump_outputs else None     # the last timed step's result
     launches = ops.total_launches()
     counts = dict(ops.launch_counts)
     passes = {k: pipe.pass_counts[k] - before[k] for k in before}
@@ -467,6 +477,13 @@ def run_ours(args):
                       f"this run measured per image: {per_image}"}
     if rank == 0:
         print(json.dumps(line))
+    if args.dump_outputs:
+        if world > 1:       # every rank's last image, in rank order
+            parts = [None] * world
+            dist.all_gather_object(parts, last_out)
+            last_out = torch.cat(parts)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"final_latents": last_out})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -509,6 +526,8 @@ def run_sweep64(args, rank, world, dev, image, host_latents, embeds_host, timed,
             "checksum_of_checksums": hashlib.sha1("".join(sums[str(sd)] for sd in seeds).encode()).hexdigest()[:16]}
     if rank == 0:
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"final_latents": full})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -738,8 +757,16 @@ def main():
                          "reference's max_refinement_steps)")
     ap.add_argument("--ref-refine", type=int, default=1,
                     help="reference arm: refinement iterations of the bounded samples after the first timed step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step (the final "
+                         "latents of its image; with --sweep64 of every seed) as DIR/final_latents.npy in float32, to "
+                         "compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the CUDA arm")
         return run_reference(args)
     return run_ours(args)
 

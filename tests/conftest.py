@@ -14,7 +14,8 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference mounted (build container only)")
+    config.addinivalue_line("markers", "reference: compares with the reference's own outputs (run live when its "
+                                       "sources are available, else as stored under tests/golden)")
 
 
 @pytest.fixture(scope="session")
