@@ -33,8 +33,7 @@ def needs_build() -> bool:
 def build(force: bool = False, verbose: bool = False) -> str:
     if not force and not needs_build():
         return OUT
-    extra = os.environ.get("GA_NVCC_EXTRA", "").split()      # experiments only (e.g. -DGA_TAIL_BWD_MIN_CTAS=8)
-    cmd = [_nvcc(), *NVCC_FLAGS, *extra, "-I", INCLUDE, "-I", CSRC, *[os.path.join(CSRC, s) for s in SOURCES], "-o", OUT]
+    cmd = [_nvcc(), *NVCC_FLAGS, "-I", INCLUDE, "-I", CSRC, *[os.path.join(CSRC, s) for s in SOURCES], "-o", OUT]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     r = subprocess.run(cmd, capture_output=True, text=True)

@@ -253,16 +253,10 @@ cross_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid
 // streams the H heads through the pipeline, so the head-sum of P stays in the two groups' registers and is combined
 // once per group through one shared staging tile, in a fixed order, then written coalesced: deterministic, no atomics.
 constexpr int kPipeThreads = 512;
-constexpr int kMaxStages = 6;   // shared-memory ring depth of the pipelined backward / grouped forward
+constexpr int kMaxStages = 6;   // shared-memory ring depth of the grouped forward and of the streaming K1 / K2
 constexpr int kFwdStages = 12;  // flat forward: Q-only stages
 constexpr int kStageCols = 256;
 constexpr int kGroupThreads = 128;
-
-#ifdef GA_DEBUG
-#define GA_ABL(p, bit) (((p).ablate & (bit)) != 0)
-#else
-#define GA_ABL(p, bit) false   // the ablation switch does not exist in release builds
-#endif
 
 struct PipeParams {
   void* o;
@@ -277,9 +271,6 @@ struct PipeParams {
   int n_sbuf;       // S/P buffers in TMEM: 4 when 4*80 + 2*npv <= 512, else 2
   int n_obuf;       // O buffers in TMEM: as many as fit behind the S buffers (2 .. 4)
   int direct_store; // 1: epilogue stores from registers (short rings), 0: staged in the dead Q tile + TMA store
-#ifdef GA_DEBUG
-  int ablate;       // debug builds only (-DGA_DEBUG, env GA_ABLATE): 1 = no O store, 2 = no exponentials, 4 = no Q loads.  WRONG RESULTS.
-#endif
   float scale;
 };
 
@@ -326,11 +317,8 @@ struct ItemIter {
   }
 };
 
-// NG softmax groups: 2 (16 warps; needed when maps are kept: the head-sum lives in the groups' registers) or 3 (20
-// warps, flat mode: the softmax groups are the busiest role of the flat kernel, a third one raises its throughput 1.5x;
-// 128 registers per softmax thread are enough without the map accumulator).
-template <int NG>
-__global__ void __launch_bounds__(128 * (NG + 2), 1)
+// Two softmax groups (16 warps): with maps kept the head-sum lives in the groups' registers, 184 per softmax thread.
+__global__ void __launch_bounds__(kPipeThreads, 1)
 cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                               const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_o,
                               const PipeParams p) {
@@ -406,9 +394,9 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
   // epilogue stores its rows straight from registers and the stage is released by the second GEMM's commit.
   const bool direct = p.direct_store != 0;
 
-  constexpr int kCtlWarp = 4 + 4 * NG;               // control warpgroup: producer, MMA issuer 1, MMA issuer 2, idle
+  constexpr int kCtlWarp = 12;                       // control warpgroup: producer, MMA issuer 1, MMA issuer 2, idle
   if (warp >= kCtlWarp) {
-    reg_dealloc<(NG == 2 ? 56 : 40)>();
+    reg_dealloc<56>();
     if (warp == kCtlWarp) {
       // ------------------------------------------------------------------------------------- TMA producer
       // Flat mode: K and V are loaded once per batch element of the CTA's range (the TMA handles one box row of <= 128
@@ -436,10 +424,9 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
         if (k >= S) mbar_wait(SMEM_FREE(ss), par ^ 1u);
         if (elect_one()) {
           const uint32_t sQ = base + ss * stage_bytes, sK = sQ + p.nblk * kQBlockBytes, sV = sK + p.nblk * kKVBlockBytes;
-          const bool load_q = !GA_ABL(p, 4);
-          mbar_expect_tx(FULL(ss), stage_bytes - (load_q ? 0u : q_bytes));
+          mbar_expect_tx(FULL(ss), stage_bytes);
           for (int blk = 0; blk < p.nblk; ++blk) {
-            if (load_q) tma_load_4d(sQ + blk * kQBlockBytes, &map_q, FULL(ss), blk * kBlockCols, it.h, it.tile * kM, it.b);
+            tma_load_4d(sQ + blk * kQBlockBytes, &map_q, FULL(ss), blk * kBlockCols, it.h, it.tile * kM, it.b);
             if (!kvres) {
               tma_load_4d(sK + blk * kKVBlockBytes, &map_k, FULL(ss), blk * kBlockCols, it.h, 0, it.b);
               tma_load_4d(sV + blk * kKVBlockBytes, &map_v, FULL(ss), blk * kBlockCols, it.h, 0, it.b);
@@ -554,7 +541,7 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
       tc_fence_after();
       const float inv = s_inv[k & 7][r];
       const uint32_t sO = base + ss * stage_bytes;    // the Q tile of this stage is dead once MMA1 has retired
-      for (int c0 = 0; c0 < p.npv / 16 && !GA_ABL(p, 8); c0 += 4) {    // up to 64 columns per TMEM round trip
+      for (int c0 = 0; c0 < p.npv / 16; c0 += 4) {    // up to 64 columns per TMEM round trip
         float ov[64];
 #pragma unroll
         for (int u = 0; u < 4; ++u)
@@ -575,7 +562,7 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
       fence_proxy_async_smem();
       __syncwarp();
       if (elect_one()) {
-        for (int blk = 0; blk < p.nblk && !GA_ABL(p, 1); ++blk)
+        for (int blk = 0; blk < p.nblk; ++blk)
           tma_store_4d(&map_o, sO + blk * kQBlockBytes + (uint32_t)warp * 4096u, blk * kBlockCols, it.h,
                        it.tile * kM + warp * 32, it.b);
         bulk_commit_group();
@@ -601,18 +588,18 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
     __syncwarp();
   } else {
     // setmaxnreg moves registers inside the CTA's OWN launch allocation (threads x registers at launch), not the SM's
-    // file: 512 x 128 = 64 K for NG == 2 (56 + 88 + 2 x 184 per 128 threads), 640 x 96 = 60 K for NG == 3
-    // (40 + 88 + 3 x 112 = 464 <= 480); asking for more spins forever in USETMAXREG.TRY_ALLOC.
-    reg_alloc<(NG == 2 ? 184 : 112)>();
+    // file: 512 x 128 = 64 K (56 + 88 + 2 x 184 per 128 threads); asking for more spins forever in
+    // USETMAXREG.TRY_ALLOC.
+    reg_alloc<184>();
     // ------------------------------------------------------------------------------------ softmax groups
-    const int g = (warp - 4) >> 2;                    // handles items k with k % NG == g
+    const int g = (warp - 4) >> 2;                    // handles items k with k % 2 == g
     const int r = ((warp & 3) << 5) + lane;           // row of the tile = TMEM lane
     const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     const float sc = p.scale * 1.4426950408889634f;
-    float pacc[NG == 2 ? kTpad : 1];                  // head-sum of P (maps kept: NG == 2 only)
-    if (NG == 2 && p.grouped) {
+    float pacc[kTpad];                                // head-sum of P (maps kept)
+    if (p.grouped) {
 #pragma unroll
-      for (int j = 0; j < (NG == 2 ? kTpad : 1); ++j) pacc[j] = 0.f;
+      for (int j = 0; j < kTpad; ++j) pacc[j] = 0.f;
     }
 
     auto process = [&](int k, int b, int h, int tile) {
@@ -620,19 +607,12 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
       const uint32_t lane_addr = lane_base + colS(k);
       mbar_wait(S_READY(sIdx(k)), sPar(k));
       tc_fence_after();
-      if (GA_ABL(p, 16)) {                           // hand the buffer straight back
-        s_inv[k & 7][r] = 1.f;
-        tc_fence_before();
-        mbar_arrive(P_READY(sIdx(k)));
-        return;
-      }
       float s[kTpad];
 #pragma unroll
       for (int cc = 0; cc < kTpad / 16; ++cc) tmem_ld16(lane_addr + cc * 16, s + cc * 16);
       tmem_ld_wait();
       float m, sum;
-      if (GA_ABL(p, 2)) { m = 0.f; sum = 1.f; }
-      else row_softmax_ilp(s, p.T, sc, m, sum);
+      row_softmax_ilp(s, p.T, sc, m, sum);
 #pragma unroll
       for (int cc = 0; cc < kTpad / 16; ++cc) {
         uint32_t packed[8];
@@ -645,11 +625,9 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
       tmem_st_wait();
       tc_fence_before();
       mbar_arrive(P_READY(sIdx(k)));
-      if constexpr (NG == 2) {
-        if (p.grouped) {
+      if (p.grouped) {
 #pragma unroll
-          for (int j = 0; j < kTpad; ++j) pacc[j] = fmaf(s[j], inv, pacc[j]);
-        }
+        for (int j = 0; j < kTpad; ++j) pacc[j] = fmaf(s[j], inv, pacc[j]);
       }
       if (row < p.N)
         p.lse[((int64_t)b * p.H + h) * p.N + row] = (m * sc + lg2_approx(sum)) * 0.6931471805599453f;
@@ -659,12 +637,12 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
     it.init(p);
     if (!p.grouped) {
       for (int i = 0; i < g; ++i) it.next(p);
-      for (int k = g; k < n_items; k += NG) {
+      for (int k = g; k < n_items; k += 2) {
         process(k, it.b, it.h, it.tile);
 #pragma unroll
-        for (int i = 0; i < NG; ++i) it.next(p);
+        for (int i = 0; i < 2; ++i) it.next(p);
       }
-    } else if constexpr (NG == 2) {
+    } else {
       int k = 0;
       for (int u = 0; u < my_units; ++u) {
         const int unit = blockIdx.x + u * gridDim.x;
@@ -710,13 +688,12 @@ cross_attn_fwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const _
 // 64-channel BLOCKS: a stage is (Q block, K block) = 26 KB, S is accumulated over the blocks as they land and a stage
 // is released by the commit that follows its own k-steps; the item's V (needed only by the second GEMM) waits in a
 // small ring of V slots; O rows leave from registers.  Softmax groups, head-sum accumulation and TMEM layout are
-// those of the pipelined kernel (NG = 2).
+// those of the pipelined kernel.
 struct FwdStreamParams {
   PipeParams b;
   int ring_stages;   // (Q block, K block) stages, 2 .. kMaxStages
   int v_slots;       // 2 .. 4
   int stage_out;     // leading 64-channel blocks of O that leave through per-warp TMA-store staging tiles (0, 1 or 2)
-  int acc_bulk;      // 1: a unit's 128 x T head-sum tile (contiguous in `acc`) leaves with one cp.async.bulk
 };
 constexpr uint32_t kOutStageBytes = 4u * 4096u;   // one staged block: 4 epilogue warps x (32 rows x 128 bytes)
 
@@ -990,60 +967,29 @@ cross_attn_fwd_tc_stream_kernel(const __grid_constant__ CUtensorMap map_q, const
           p.lse[((int64_t)b * p.H + h) * p.N + row] = (m * sc + lg2_approx(sum)) * 0.6931471805599453f;
       }
       // ---- end of the (b, tile) unit: combine the two groups' head sums and write the accumulator rows
-      if (sp.acc_bulk) {
-        // The unit's rows are CONTIGUOUS in `acc` (128 rows x T floats): the tile is assembled densely in shared memory
-        // (row stride T = 77: odd, conflict-free) and leaves with ONE bulk copy issued by one thread, instead of eight
-        // warps looping over dependent shared-load / global-store pairs (the loop and its barrier were ~15 % of the
-        // softmax groups' stall samples).  Group 1 does not wait for the copy: it only waits, at the NEXT unit, for the
-        // tile to have been read.
-        const bool t0 = tid == kGroupThreads;                  // first thread of group 0 owns the bulk group
-        if (u > 0 && t0) bulk_wait_read0();
-        named_bar_sync(1, 2 * kGroupThreads);
-        if (g == 1) {
+      if (g == 1) {
 #pragma unroll
-          for (int j = 0; j < kTpad; ++j)
-            if (j < p.T) sAcc[r * p.T + j] = pacc[j];
-          named_bar_arrive(2, 2 * kGroupThreads);
-        } else {
-          named_bar_sync(2, 2 * kGroupThreads);
-#pragma unroll
-          for (int j = 0; j < kTpad; ++j)
-            if (j < p.T) sAcc[r * p.T + j] += pacc[j];
-          fence_proxy_async_smem();
-          named_bar_sync(3, kGroupThreads);
-          if (t0) {
-            const int rows = min(kM, p.N - tile * kM);
-            bulk_store_1d(p.acc + ((int64_t)b * p.N + (int64_t)tile * kM) * p.T, smem_u32(sAcc),
-                          (uint32_t)(rows * p.T * (int)sizeof(float)));
-            bulk_commit_group();
-          }
-        }
-      } else {
-        if (g == 1) {
-#pragma unroll
-          for (int j = 0; j < kTpad; ++j) sAcc[r * kAccStride + j] = pacc[j];
-        }
-        named_bar_sync(1, 2 * kGroupThreads);
-        if (g == 0) {
-#pragma unroll
-          for (int j = 0; j < kTpad; ++j) sAcc[r * kAccStride + j] += pacc[j];
-        }
-        named_bar_sync(2, 2 * kGroupThreads);
-        for (int i = warp - 4; i < kM; i += 8) {
-          const int gr = tile * kM + i;
-          if (gr >= p.N) break;
-#pragma unroll
-          for (int kk = 0; kk < 3; ++kk) {
-            const int j = lane + 32 * kk;
-            if (j < p.T) p.acc[((int64_t)b * p.N + gr) * p.T + j] = sAcc[i * kAccStride + j];
-          }
-        }
-        named_bar_sync(3, 2 * kGroupThreads);
+        for (int j = 0; j < kTpad; ++j) sAcc[r * kAccStride + j] = pacc[j];
       }
+      named_bar_sync(1, 2 * kGroupThreads);
+      if (g == 0) {
+#pragma unroll
+        for (int j = 0; j < kTpad; ++j) sAcc[r * kAccStride + j] += pacc[j];
+      }
+      named_bar_sync(2, 2 * kGroupThreads);
+      for (int i = warp - 4; i < kM; i += 8) {
+        const int gr = tile * kM + i;
+        if (gr >= p.N) break;
+#pragma unroll
+        for (int kk = 0; kk < 3; ++kk) {
+          const int j = lane + 32 * kk;
+          if (j < p.T) p.acc[((int64_t)b * p.N + gr) * p.T + j] = sAcc[i * kAccStride + j];
+        }
+      }
+      named_bar_sync(3, 2 * kGroupThreads);
 #pragma unroll
       for (int j = 0; j < kTpad; ++j) pacc[j] = 0.f;
     }
-    if (sp.acc_bulk && tid == kGroupThreads) bulk_wait_all0();     // the last tile has left before the CTA exits
   }
   tc_fence_before();
   __syncthreads();
@@ -1207,12 +1153,25 @@ cross_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid
   if (warp == 0) tmem_dealloc(tmem, (uint32_t)p.tmem_cols);
 }
 
-// ============================================================================ K2, persistent pipelined variant
-// Same warpgroup roles as the pipelined forward.  Per item: TMA brings Q, dO, K, V; the MMA warp issues S = QK^T and
-// dP = dO V^T back to back into two TMEM regions; a compute group turns them into dS (16-bit, written over S); the MMA
-// warp issues dQ = dS K (K as the MN-major B operand); the epilogue warpgroup converts dQ, stages it in the item's dead
-// Q tile and hands it to the TMA.  dQ has its own TMEM columns when they fit (d <= 80), so the next item's first two
-// GEMMs never wait for an epilogue.
+// =================================================================================== K2, persistent STREAMING kernel
+// One persistent CTA per SM with the warpgroup roles of the pipelined forward; the work items are the B * tiles row
+// tiles of one head, split into contiguous ranges over teams of H CTAs (the forward's flat split).  Per item the first
+// MMA warp issues S = Q K^T and dP = dO V^T into two TMEM regions, a compute group turns them into dS (16-bit, written
+// over S), the second MMA warp issues dQ = dS K (K as the MN-major B operand) and the epilogue warpgroup converts dQ.
+// What the shared memory holds is chosen so that the producer never waits for an epilogue (a ring of whole items --
+// Q, dO, K, V of one 128-row tile: 104 KB per stage at d = 80, 156 KB at d = 160 -- left the SM with too few bytes in
+// flight: DRAM 25-34 %, issue slots 12-19 %, tensor pipe 8-9 %, profiles/r02_ncu_summary.json):
+//   * K and V of the current (batch element, head) live in two dedicated slots (the next element's K/V are fetched
+//     into the other slot while the current one is in use); a CTA's items are consecutive row tiles of one head, so
+//     they change rarely;
+//   * the ring holds 64-channel BLOCKS of Q and dO (32 KB per stage: 4 stages at d = 80, 3 at d = 160).  S and dP
+//     are accumulated over the blocks as they arrive, and a stage is released by the tcgen05.commit that follows
+//     ITS OWN k-steps -- the producer streams Q / dO at HBM rate instead of waiting for epilogues;
+//   * dQ rows leave from registers.
+// TMEM: three stages of 160 columns (S | dP, dQ over dP) when npv <= 80, else two stages of 256 columns, so a compute
+// group finds the GEMM outputs of its next item ready when it finishes one.  S and dP of item k overwrite the columns
+// of dS(k - nT), and of dQ(k - nT) when dQ lies over dP: the first MMA warp waits for that item's dQ GEMM (DQ_READY)
+// and, in the aliased case, for its epilogue (TMEM_FREE).
 struct BwdPipeParams {
   void* d_q;
   const float* lse;
@@ -1221,323 +1180,12 @@ struct BwdPipeParams {
   int d_acc_rstride;
   int B, H, N, T, d;
   int nblk, npv, bf16;
-  int tiles, units, smem_stages;
+  int tiles, units;
+  float scale;
+  // col_dq and tstages are read together: at an 8-byte aligned offset they come in with one 64-bit constant load
   int col_dq;          // TMEM column of dQ inside a stage: 160 (own columns) or 80 (over dP)
   int tstages;         // TMEM stages: 3 (160 columns each, dQ over dP) when npv <= 80, else 2 (256 columns each)
-  int direct_store;    // 1: dQ rows stored from registers (short rings), 0: staged + TMA store
-  float scale;
 };
-
-__global__ void __launch_bounds__(kPipeThreads, 1)
-cross_attn_bwd_tc_pipe_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_do,
-                              const __grid_constant__ CUtensorMap map_k, const __grid_constant__ CUtensorMap map_v,
-                              const __grid_constant__ CUtensorMap map_dq, const BwdPipeParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t bars[24];   // full[6], smem_free[6], then sd_ready / ds_ready / dq_ready / tmem_free x 3
-  __shared__ uint32_t tmem_base_slot;
-
-  const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t stage_bytes = (uint32_t)p.nblk * 2u * (kQBlockBytes + kKVBlockBytes);
-  auto FULL = [&](int s) { return smem_u32(&bars[s]); };
-  auto SMEM_FREE = [&](int s) { return smem_u32(&bars[kMaxStages + s]); };
-  auto SD_READY = [&](int s) { return smem_u32(&bars[2 * kMaxStages + s]); };
-  auto DS_READY = [&](int s) { return smem_u32(&bars[2 * kMaxStages + 3 + s]); };
-  auto DQ_READY = [&](int s) { return smem_u32(&bars[2 * kMaxStages + 6 + s]); };
-  auto TMEM_FREE = [&](int s) { return smem_u32(&bars[2 * kMaxStages + 9 + s]); };
-  // TMEM stages: nT = 3 stages of 160 columns (S | dP, dQ over dP) when dQ fits in dP's 80 columns (d <= 80), else two
-  // stages of 256 columns.  With three stages a compute group finds the GEMM outputs of its next item ready when it
-  // finishes one (see the forward kernel).
-  const int nT = p.tstages;
-  const uint32_t stage_cols = nT == 3 ? 160u : (uint32_t)kStageCols;
-  auto tIdx = [&](int k) { return nT == 3 ? k % 3 : (k & 1); };
-  auto tPar = [&](int k) { return (uint32_t)(nT == 3 ? k / 3 : k >> 1) & 1u; };
-  // flat work split of the forward kernel: teams of H CTAs own contiguous ranges of the B * tiles row tiles
-  const int teams = gridDim.x / p.H, team = blockIdx.x / p.H, my_h = blockIdx.x % p.H;
-  const int rt0 = (int)(((int64_t)p.units * team) / teams);
-  const int n_items = (int)(((int64_t)p.units * (team + 1)) / teams) - rt0;
-  const bool dq_aliased = p.col_dq == kColDP;
-
-  if (tid == 0) {
-    prefetch_tmap(&map_q); prefetch_tmap(&map_do); prefetch_tmap(&map_k); prefetch_tmap(&map_v); prefetch_tmap(&map_dq);
-    for (int s = 0; s < kMaxStages; ++s) { mbar_init(FULL(s), 1); mbar_init(SMEM_FREE(s), p.direct_store ? 1 : 4); }
-    for (int s = 0; s < 3; ++s) {
-      mbar_init(SD_READY(s), 1);
-      mbar_init(DS_READY(s), kGroupThreads);
-      mbar_init(DQ_READY(s), 1);
-      mbar_init(TMEM_FREE(s), kGroupThreads);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 0) tmem_alloc(smem_u32(&tmem_base_slot), 512u);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = uniform_u32(tmem_base_slot);
-  const int fmt = p.bf16 ? 1 : 0;
-  const int ksteps = (p.d + 15) >> 4;
-  const int S = p.smem_stages;
-  const bool bf16 = p.bf16 != 0;
-  const bool direct = p.direct_store != 0;          // see the forward kernel
-
-  auto coords = [&](int k, int& b, int& h, int& tile) {
-    const int rt = rt0 + k;
-    h = my_h;
-    b = rt / p.tiles;
-    tile = rt - b * p.tiles;
-  };
-
-  if (warp >= 12) {
-    reg_dealloc<56>();
-    if (warp == 12) {
-      // TMA producer (warp-uniform, one elected lane issues); K and V are re-loaded only when the stage's batch element
-      // changes (see the forward kernel)
-      int kv_tag[kMaxStages] = {-1, -1, -1, -1, -1, -1};
-      int ss = 0;
-      uint32_t par = 0;
-      const uint32_t qg_bytes = 2u * (uint32_t)p.nblk * kQBlockBytes;
-      for (int k = 0; k < n_items; ++k) {
-        int b, h, tile;
-        coords(k, b, h, tile);
-        if (k >= S) mbar_wait(SMEM_FREE(ss), par ^ 1u);
-        const bool with_kv = kv_tag[ss] != b;
-        kv_tag[ss] = b;
-        if (elect_one()) {
-          const uint32_t sQ = base + ss * stage_bytes, sG = sQ + p.nblk * kQBlockBytes, sK = sG + p.nblk * kQBlockBytes,
-                         sV = sK + p.nblk * kKVBlockBytes;
-          mbar_expect_tx(FULL(ss), with_kv ? stage_bytes : qg_bytes);
-          for (int blk = 0; blk < p.nblk; ++blk) {
-            tma_load_4d(sQ + blk * kQBlockBytes, &map_q, FULL(ss), blk * kBlockCols, h, tile * kM, b);
-            tma_load_4d(sG + blk * kQBlockBytes, &map_do, FULL(ss), blk * kBlockCols, h, tile * kM, b);
-            if (with_kv) {
-              tma_load_4d(sK + blk * kKVBlockBytes, &map_k, FULL(ss), blk * kBlockCols, h, 0, b);
-              tma_load_4d(sV + blk * kKVBlockBytes, &map_v, FULL(ss), blk * kBlockCols, h, 0, b);
-            }
-          }
-        }
-        __syncwarp();
-        if (++ss == S) { ss = 0; par ^= 1u; }
-      }
-    } else if (warp == 13) {
-      // MMA issuer 1: S = Q K^T and dP = dO V^T (two issuer warps, see the forward kernel).  Its outputs overwrite the
-      // columns dS(k-2) lives in (and dQ(k-2) when dQ aliases dP): wait for MMA3(k-2) to complete (DQ_READY) and, if
-      // aliased, for the epilogue of k-2 (TMEM_FREE).
-      const uint32_t idesc_nt = make_idesc(fmt, 0, kTpad, kM);
-      const uint32_t oG = p.nblk * kQBlockBytes, oK = 2u * p.nblk * kQBlockBytes, oV = oK + p.nblk * kKVBlockBytes;
-      const uint64_t dQ0 = smem_desc_sw128(base, 16, 1024), dG0 = smem_desc_sw128(base + oG, 16, 1024);
-      const uint64_t dK0 = smem_desc_sw128(base + oK, 16, 1024), dV0 = smem_desc_sw128(base + oV, 16, 1024);
-      int ss = 0;
-      uint32_t par = 0;
-      for (int k = 0; k < n_items; ++k) {
-        const int ts = tIdx(k);
-        const uint32_t ph = tPar(k);
-        if (k >= nT) {
-          mbar_wait(DQ_READY(ts), ph ^ 1u);
-          if (dq_aliased) mbar_wait(TMEM_FREE(ts), ph ^ 1u);
-        }
-        mbar_wait(FULL(ss), par);
-        tc_fence_after();
-        if (elect_one()) {
-          issue_kmajor_gemm(tmem + ts * stage_cols + kColS, desc_advance(dQ0, ss * stage_bytes), kQBlockBytes,
-                            desc_advance(dK0, ss * stage_bytes), kKVBlockBytes, ksteps, idesc_nt);
-          issue_kmajor_gemm(tmem + ts * stage_cols + kColDP, desc_advance(dG0, ss * stage_bytes), kQBlockBytes,
-                            desc_advance(dV0, ss * stage_bytes), kKVBlockBytes, ksteps, idesc_nt);
-          tc_commit(SD_READY(ts));
-        }
-        __syncwarp();
-        if (++ss == S) { ss = 0; par ^= 1u; }
-      }
-    } else if (warp == 14) {
-      // MMA issuer 2: dQ = dS K
-      const uint32_t idesc_dq = make_idesc(fmt, 1, p.npv, kM);
-      const uint32_t oK = 2u * p.nblk * kQBlockBytes;
-      const uint64_t dKmn0 = smem_desc_sw128(base + oK, kKVBlockBytes, 1024);
-      int ss = 0;
-      for (int k = 0; k < n_items; ++k) {
-        const int ts = tIdx(k);
-        const uint32_t ph = tPar(k);
-        mbar_wait(DS_READY(ts), ph);
-        if (!dq_aliased && k >= nT) mbar_wait(TMEM_FREE(ts), ph ^ 1u);
-        tc_fence_after();
-        if (elect_one()) {
-          issue_tmem_gemm(tmem + ts * stage_cols + p.col_dq, tmem + ts * stage_cols + kColP,
-                          desc_advance(dKmn0, ss * stage_bytes), kTpad / 16, idesc_dq, false);
-          tc_commit(DQ_READY(ts));
-          if (direct) tc_commit(SMEM_FREE(ss));
-        }
-        __syncwarp();
-        if (++ss == S) ss = 0;
-      }
-    }
-  } else if (warp < 4) {
-    reg_dealloc<88>();
-    // ---------------------------------------------------------------------------------------- epilogue (dQ)
-    // four independent warps, one 32-row TMA store each (see the forward kernel)
-    const int r = (warp << 5) + lane;
-    const uint32_t lane_base = tmem + ((uint32_t)(warp * 32) << 16);
-    int ss = 0;
-    if (direct) {
-      // short rings: rows go from registers to global memory (the stage was handed back by MMA3's commit)
-      for (int k = 0; k < n_items; ++k) {
-        const int ts = tIdx(k);
-        mbar_wait(DQ_READY(ts), tPar(k));
-        tc_fence_after();
-        int b, h, tile;
-        coords(k, b, h, tile);
-        const int row = tile * kM + r;
-        uint8_t* grow = reinterpret_cast<uint8_t*>(p.d_q) + (((int64_t)b * p.N + row) * p.H + h) * (int64_t)p.d * 2;
-        for (int cc = 0; cc < p.npv / 16; ++cc) {
-          float ov[16];
-          tmem_ld16(lane_base + ts * stage_cols + p.col_dq + cc * 16, ov);
-          tmem_ld_wait();
-          if (row < p.N) {
-            uint32_t w[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) w[i] = pack16(ov[2 * i], ov[2 * i + 1], bf16);
-            const int col = cc * 16;
-            if (col < p.d) *reinterpret_cast<uint4*>(grow + col * 2) = make_uint4(w[0], w[1], w[2], w[3]);
-            if (col + 8 < p.d) *reinterpret_cast<uint4*>(grow + col * 2 + 16) = make_uint4(w[4], w[5], w[6], w[7]);
-          }
-        }
-        tc_fence_before();
-        mbar_arrive(TMEM_FREE(ts));
-      }
-    }
-    for (int k = 0; k < n_items && !direct; ++k) {
-      const int ts = tIdx(k);
-      const uint32_t ph = tPar(k);
-      mbar_wait(DQ_READY(ts), ph);
-      tc_fence_after();
-      const uint32_t sO = base + ss * stage_bytes;    // the Q tile of this stage: dead since S = Q K^T retired
-      for (int c0 = 0; c0 < p.npv / 16; c0 += 4) {
-        float ov[64];
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-          if (c0 + u < p.npv / 16) tmem_ld16(lane_base + ts * stage_cols + p.col_dq + (c0 + u) * 16, ov + u * 16);
-        tmem_ld_wait();
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          if (c0 + u < p.npv / 16) {
-            uint32_t w[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) w[i] = pack16(ov[u * 16 + 2 * i], ov[u * 16 + 2 * i + 1], bf16);
-            st_swizzled_32B(sO + (uint32_t)((c0 + u) >> 2) * kQBlockBytes, r, ((c0 + u) & 3) * 2, w);
-          }
-        }
-      }
-      tc_fence_before();
-      mbar_arrive(TMEM_FREE(ts));
-      fence_proxy_async_smem();
-      __syncwarp();
-      int b, h, tile;
-      coords(k, b, h, tile);
-      if (elect_one()) {
-        for (int blk = 0; blk < p.nblk; ++blk)
-          tma_store_4d(&map_dq, sO + blk * kQBlockBytes + (uint32_t)warp * 4096u, blk * kBlockCols, h, tile * kM + warp * 32,
-                       b);
-        bulk_commit_group();
-        if (S < 5) {
-          bulk_wait_read0();
-          mbar_arrive(SMEM_FREE(ss));
-        } else if (k >= 1) {
-          bulk_wait_read1();
-          mbar_arrive(SMEM_FREE(ss == 0 ? S - 1 : ss - 1));
-        }
-      }
-      __syncwarp();
-      if (++ss == S) ss = 0;
-    }
-    if (!direct && elect_one()) {
-      bulk_wait_read0();
-      if (n_items >= 1 && S >= 5) mbar_arrive(SMEM_FREE(ss == 0 ? S - 1 : ss - 1));
-      bulk_wait_all0();
-    }
-    __syncwarp();
-  } else {
-    reg_alloc<184>();
-    const int g = (warp - 4) >> 2;
-    const int r = ((warp & 3) << 5) + lane;
-    const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-    const float sc = p.scale * 1.4426950408889634f;
-    for (int k = g; k < n_items; k += 2) {
-      int b, h, tile;
-      coords(k, b, h, tile);
-      const int row = tile * kM + r;
-      const bool live = row < p.N;
-      const int ts = tIdx(k);
-      const uint32_t ph = tPar(k);
-      const uint32_t lane_addr = lane_base + ts * stage_cols;
-      // issue the row's LSE load before waiting for the GEMMs
-      const float l2 = live ? __ldg(p.lse + ((int64_t)b * p.H + h) * p.N + row) * 1.4426950408889634f : 0.f;
-      const float* dacc = (p.d_acc != nullptr && live)
-                              ? p.d_acc + (int64_t)b * p.d_acc_bstride + (int64_t)row * p.d_acc_rstride : nullptr;
-      mbar_wait(SD_READY(ts), ph);
-      tc_fence_after();
-      float s[kTpad], dp[kTpad];
-#pragma unroll
-      for (int cc = 0; cc < kTpad / 16; ++cc) {
-        tmem_ld16(lane_addr + kColS + cc * 16, s + cc * 16);
-        tmem_ld16(lane_addr + kColDP + cc * 16, dp + cc * 16);
-      }
-      tmem_ld_wait();
-      if (dacc != nullptr) {
-        if ((p.d_acc_rstride & 3) == 0) {          // 16-byte aligned rows (the tail kernel pads them to 80 floats)
-#pragma unroll
-          for (int j = 0; j < kTpad; j += 4) {
-            if (j + 3 < p.d_acc_rstride) {
-              const float4 v4 = __ldg(reinterpret_cast<const float4*>(dacc + j));
-              dp[j] += v4.x; dp[j + 1] += v4.y; dp[j + 2] += v4.z; dp[j + 3] += v4.w;
-            }
-          }
-        } else {
-#pragma unroll
-          for (int j = 0; j < kTpad; ++j)
-            if (j < p.T) dp[j] += __ldg(dacc + j);
-        }
-      }
-      float d4[4] = {0.f, 0.f, 0.f, 0.f};          // four independent chains for rowsum(P o dP)
-#pragma unroll
-      for (int j = 0; j < kTpad; ++j) {
-        const bool ok = live && (j < kTpad - 16 || j < p.T);
-        const float pr = ok ? ex2_approx(fmaf(s[j], sc, -l2)) : 0.f;
-        s[j] = pr;
-        d4[j & 3] = fmaf(pr, dp[j], d4[j & 3]);
-      }
-      const float dsum = (d4[0] + d4[1]) + (d4[2] + d4[3]);
-#pragma unroll
-      for (int cc = 0; cc < kTpad / 16; ++cc) {
-        uint32_t packed[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int j = cc * 16 + 2 * i;
-          packed[i] = pack16(s[j] * (dp[j] - dsum) * p.scale, s[j + 1] * (dp[j + 1] - dsum) * p.scale, bf16);
-        }
-        tmem_st8(lane_addr + kColP + cc * 8, packed);
-      }
-      tmem_st_wait();
-      tc_fence_before();
-      mbar_arrive(DS_READY(ts));
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem, 512u);
-}
-
-// ====================================================================== K2, persistent STREAMING variant (d > 64)
-// The pipelined kernel above keeps whole items (Q, dO, K, V of one 128-row tile) in its shared-memory ring: 104 KB per
-// stage at d = 80 and 156 KB at d = 160, i.e. two stages / one stage, and a stage is only handed back when the item's
-// LAST GEMM has retired.  ncu on that kernel (profiles/r02_ncu_summary.json): DRAM 25-34 %, issue slots 12-19 %,
-// tensor pipe 8-9 % -- nothing is busy, the SM simply has too few bytes in flight.  This variant changes what the ring
-// holds:
-//   * K and V of the current (batch element, head) live in two dedicated slots (the next element's K/V are fetched
-//     into the other slot while the current one is in use); a CTA's items are consecutive row tiles of one head, so
-//     they change rarely;
-//   * the ring holds 64-channel BLOCKS of Q and dO (32 KB per stage: 4 stages at d = 80, 3 at d = 160).  S and dP
-//     are accumulated over the blocks as they arrive, and a stage is released by the tcgen05.commit that follows
-//     ITS OWN k-steps -- the producer streams Q / dO at HBM rate instead of waiting for epilogues;
-//   * dQ rows leave from registers (the dead-Q-tile staging of the pipelined kernel no longer exists).
-// Compute groups, TMEM stages and the epilogue are those of the pipelined kernel.
 struct BwdStreamParams {
   BwdPipeParams b;
   int ring_stages;   // 2 .. kMaxStages
@@ -1885,27 +1533,6 @@ static int heads_per_cta_for(int H) {
   return H;
 }
 
-// GA_DISABLE_TCGEN05=1 makes AUTO pick the SIMT variant everywhere (debugging aid: A/B the two variants)
-static bool tc_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("GA_DISABLE_TCGEN05");
-    on = (e != nullptr && e[0] == '1') ? 0 : 1;
-  }
-  return on == 1;
-}
-
-
-// GA_TC_PIPE=0/1 forces the single-shot / persistent variant (debugging and A/B measurements)
-static int pipe_override() {
-  static int v = -2;
-  if (v == -2) {
-    const char* e = getenv("GA_TC_PIPE");
-    v = (e == nullptr) ? -1 : (e[0] == '1' ? 1 : 0);
-  }
-  return v;
-}
-
 static int fwd_pipe(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv, const FwdParams& f, int dtype,
                     cudaStream_t st) {
   PipeParams p;
@@ -1917,36 +1544,15 @@ static int fwd_pipe(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensor
   p.units = f.B * p.tiles;
   p.n_sbuf = (4 * kTpad + 2 * p.npv <= 512) ? 4 : 2;
   p.n_obuf = (512 - p.n_sbuf * kTpad) / p.npv >= 4 ? 4 : 2;
-#ifdef GA_DEBUG
-  {
-    const char* e = getenv("GA_ABLATE");
-    p.ablate = e != nullptr ? atoi(e) : 0;
-  }
-#endif
-  // maps kept and more than one 64-channel block: the streaming variant (GA_K1_STREAM=0 keeps the whole-item ring,
-  // =1 streams d <= 64 as well)
-  static int stream_mode = -2;
-  if (stream_mode == -2) {
-    const char* es = getenv("GA_K1_STREAM");
-    stream_mode = es == nullptr ? -1 : atoi(es);
-  }
-  if (p.grouped && ((stream_mode == -1 && p.nblk >= 2) || stream_mode == 1)) {
+  // maps kept and more than one 64-channel block: the streaming variant
+  if (p.grouped && p.nblk >= 2) {
     FwdStreamParams sp;
     sp.b = p;
     const size_t acc_bytes = (size_t)kM * kAccStride * sizeof(float), ring = (size_t)kQBlockBytes + kKVBlockBytes;
     const size_t vslot = (size_t)p.nblk * kKVBlockBytes;
-    sp.v_slots = 3;
     // O staging tiles (TMA stores instead of row-strided 16-byte stores, see the epilogue) are paid for with the third
     // V slot where needed, never with a ring stage.  Measured on B200 (profiles/r02d_k1_stage_ab.txt): d = 80
     // 210 -> 167-171 us with one staged block, d = 160 191 -> 170 us with one staged block and two V slots, 158 us with two.
-    // GA_K1_STAGE_OUT=<blocks> / GA_K1_V_SLOTS=<n> override the choice (A/B measurements).
-    static int stage_mode = -2, slot_mode = -2;
-    if (stage_mode == -2) {
-      const char* eo = getenv("GA_K1_STAGE_OUT");
-      stage_mode = eo == nullptr ? -1 : atoi(eo);
-      const char* ev = getenv("GA_K1_V_SLOTS");
-      slot_mode = ev == nullptr ? -1 : atoi(ev);
-    }
     // dynamic + static shared memory (barriers, s_inv: 4.4 KB) must stay within the 227 KB a CTA can opt in to
     auto stages_for = [&](int blocks, int v_slots) {
       for (int n = kMaxStages; n >= 2; --n)
@@ -1956,33 +1562,19 @@ static int fwd_pipe(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensor
     const int without = stages_for(0, 3);
     sp.stage_out = 0;
     sp.v_slots = 3;
-    if (stage_mode < 0) {
-      // first fit that keeps the ring depth: two staged blocks only when two FULL 64-channel blocks exist (staging the
-      // 16-channel tail of d = 80 at the price of a V slot measured slower: 176 vs 171 us)
-      const int full_blocks = p.d / kBlockCols;
-      const int cand[4][2] = {{2, 3}, {2, 2}, {1, 3}, {1, 2}};
-      for (int i = 0; i < 4; ++i) {
-        if (cand[i][0] == 2 && full_blocks < 2) continue;
-        if (stages_for(cand[i][0], cand[i][1]) == without) {
-          sp.stage_out = cand[i][0];
-          sp.v_slots = cand[i][1];
-          break;
-        }
+    // first fit that keeps the ring depth: two staged blocks only when two FULL 64-channel blocks exist (staging the
+    // 16-channel tail of d = 80 at the price of a V slot measured slower: 176 vs 171 us)
+    const int full_blocks = p.d / kBlockCols;
+    const int cand[4][2] = {{2, 3}, {2, 2}, {1, 3}, {1, 2}};
+    for (int i = 0; i < 4; ++i) {
+      if (cand[i][0] == 2 && full_blocks < 2) continue;
+      if (stages_for(cand[i][0], cand[i][1]) == without) {
+        sp.stage_out = cand[i][0];
+        sp.v_slots = cand[i][1];
+        break;
       }
-    } else {
-      sp.stage_out = stage_mode > 2 ? 2 : stage_mode;
     }
-    if (slot_mode == 2 || slot_mode == 3) sp.v_slots = slot_mode;
     sp.ring_stages = stages_for(sp.stage_out, sp.v_slots);
-    // one bulk copy per head-sum tile needs 16-byte aligned, 16-byte sized tiles: N % 4 == 0 and an aligned accumulator
-    static int bulk_mode = -2;
-    if (bulk_mode == -2) {
-      const char* eb = getenv("GA_K1_ACC_BULK");
-      bulk_mode = eb == nullptr ? -1 : atoi(eb);
-    }
-    // Measured SLOWER than the eight-warp write loop (d = 80: 184 vs 173 us, d = 160: 161 vs 159 us, B = 16: 17.8 vs 15.6 us;
-    // profiles/r02d_k1_stage_ab.txt): kept behind GA_K1_ACC_BULK=1 as a recorded negative result, off by default.
-    sp.acc_bulk = (bulk_mode == 1 && f.N % 4 == 0 && (reinterpret_cast<uintptr_t>(f.acc) & 15) == 0) ? 1 : 0;
     if (sp.ring_stages >= p.nblk) {
       const size_t smem_s = 1024 + acc_bytes + (size_t)sp.stage_out * kOutStageBytes + sp.v_slots * vslot + sp.ring_stages * ring;
       cudaError_t es2 = ensure_smem(reinterpret_cast<const void*>(cross_attn_fwd_tc_stream_kernel), 6, smem_s);
@@ -2007,7 +1599,7 @@ static int fwd_pipe(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensor
   const size_t smem = p.smem_stages * stage + extra;
   if (smem > 224 * 1024) return fail(GA_ERR_UNSUPPORTED, "tcgen05 pipelined cross-attention: %zu B of shared memory", smem);
   p.direct_store = p.smem_stages < 4 ? 1 : 0;
-  cudaError_t e = ensure_smem(reinterpret_cast<const void*>(cross_attn_fwd_tc_pipe_kernel<2>), 2, smem);
+  cudaError_t e = ensure_smem(reinterpret_cast<const void*>(cross_attn_fwd_tc_pipe_kernel), 2, smem);
   if (e != cudaSuccess) return fail(GA_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   int grid;
   if (p.grouped) {
@@ -2018,28 +1610,14 @@ static int fwd_pipe(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensor
     if (teams > p.units) teams = p.units;
     grid = teams * f.H;
   }
-  // GA_TC_GROUPS=3 selects the three-softmax-group variant in flat mode (d <= 64).  Measured SLOWER than two groups
-  // (3 445 vs 3 629 GB/s at B=128, N=4096, d=40): the softmax groups are not what bounds the flat kernel.  Kept for A/B runs.
-  static int force_groups = -1;
-  if (force_groups < 0) {
-    const char* e3 = getenv("GA_TC_GROUPS");
-    force_groups = e3 != nullptr ? atoi(e3) : 0;
-  }
-  const bool three = !p.grouped && p.nblk == 1 && force_groups == 3;
-  if (three) {
-    e = ensure_smem(reinterpret_cast<const void*>(cross_attn_fwd_tc_pipe_kernel<3>), 4, smem);
-    if (e != cudaSuccess) return fail(GA_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    cross_attn_fwd_tc_pipe_kernel<3><<<grid, 128 * 5, smem, st>>>(mq, mk, mv, mo, p);
-  } else {
-    cross_attn_fwd_tc_pipe_kernel<2><<<grid, 128 * 4, smem, st>>>(mq, mk, mv, mo, p);
-  }
+  cross_attn_fwd_tc_pipe_kernel<<<grid, kPipeThreads, smem, st>>>(mq, mk, mv, mo, p);
   return check_launch("cross_attn_fwd_tc_pipe");
 }
 
 bool supports_fwd(int dtype, int n_ctx, int head_dim, int heads, bool with_acc) {
   (void)heads; (void)with_acc;
   // the row softmax predicates only the last 16 of the 80 key columns on n_ctx: 65..80 keys (SD: 77)
-  return tc_enabled() && (dtype == GA_F16 || dtype == GA_BF16) && n_ctx > kTpad - 16 && n_ctx <= kTpad &&
+  return (dtype == GA_F16 || dtype == GA_BF16) && n_ctx > kTpad - 16 && n_ctx <= kTpad &&
          head_dim % 8 == 0 && head_dim >= 8 && head_dim <= 256;
 }
 bool supports_bwd(int dtype, int n_ctx, int head_dim, int heads, bool with_dkv) {
@@ -2079,7 +1657,6 @@ int fwd(const void* q, const void* k, const void* v, void* o, float* lse, float*
     // B = 2 at 32x32, the CFG pass: 14.6 vs 17.4 us -- profiles/r02d_crossover_sweep.jsonl)
     const int min_units = acc != nullptr ? (tiles >= 2 ? 16 : 24) : 2 * sm_count();
     bool use_pipe = d <= 160 && units >= min_units;
-    if (pipe_override() >= 0) use_pipe = pipe_override() == 1 && d <= 160;
     if (force_variant == 0) use_pipe = false;
     if (force_variant == 1) {
       if (d > 160) return fail(GA_ERR_UNSUPPORTED, "pipelined tcgen05 cross-attention needs head_dim <= 160");
@@ -2126,88 +1703,57 @@ int bwd(const void* q, const void* k, const void* v, const float* lse, const voi
   // items (N = 1024 d = 80: 10.9 vs 12.3 us, N = 256 d = 160: 15.0 vs 21.3 us), a tie at 128
   const int min_items = d_acc != nullptr ? (5 * sm_count()) / 4 : 2 * sm_count();
   bool use_pipe = d <= 160 && units >= min_items && H <= sm_count();
-  if (pipe_override() >= 0) use_pipe = pipe_override() == 1 && d <= 160;
   if (force_variant == 0) use_pipe = false;
   if (force_variant == 1) {
     if (d > 160) return fail(GA_ERR_UNSUPPORTED, "pipelined tcgen05 cross-attention needs head_dim <= 160");
     use_pipe = true;
   }
   if (use_pipe) {
-    BwdPipeParams p;
+    // the streaming kernel -- K/V slots + a ring of Q/dO blocks -- measured faster than a ring of whole items at every
+    // head dim (B200, profiles/r02_microbench_k2_stream.jsonl: d = 80: 386 vs 490 us, d = 160: 347 vs 419 us,
+    // d = 40: 304 vs 320 us)
+    BwdStreamParams sp;
+    BwdPipeParams& p = sp.b;
     p.d_q = d_q; p.lse = lse; p.d_acc = d_acc; p.d_acc_bstride = d_acc_bstride; p.d_acc_rstride = d_acc_rstride;
     p.B = B; p.H = H; p.N = N; p.T = T; p.d = d;
     p.nblk = nblk; p.npv = npv; p.bf16 = dtype == GA_BF16; p.scale = scale;
     p.tiles = tiles; p.units = B * tiles;      // row tiles, split over teams of H CTAs
     p.tstages = npv <= kTpad ? 3 : 2;
     p.col_dq = p.tstages == 3 ? kColDP : ((2 * kTpad + npv <= kStageCols) ? 2 * kTpad : kColDP);
-    const size_t stage = (size_t)nblk * 2 * (kQBlockBytes + kKVBlockBytes);
-    // the streaming variant -- K/V slots + a ring of Q/dO blocks -- measured faster than the whole-item ring at every
-    // head dim (B200, profiles/r02_microbench_k2_stream.jsonl: d = 80: 386 vs 490 us, d = 160: 347 vs 419 us,
-    // d = 40: 304 vs 320 us); GA_K2_STREAM=0 keeps the whole-item ring for A/B runs
-    static int stream_mode = -2;
-    if (stream_mode == -2) {
-      const char* es = getenv("GA_K2_STREAM");
-      stream_mode = es == nullptr ? -1 : atoi(es);
+    const size_t kv = (size_t)2 * 2 * nblk * kKVBlockBytes, ring = (size_t)2 * kQBlockBytes;
+    auto stages_for = [&](size_t extra) {
+      for (int n = kMaxStages; n >= 2; --n)
+        if (1024 + kv + extra + n * ring <= 226 * 1024) return n;
+      return 0;
+    };
+    // TMA-staged map-gradient tile (40 KB) whenever the rows can be described to the TMA (16-byte aligned base and
+    // strides, at most 80 columns) and two ring stages remain: d = 160 runs 242 us with two stages + the staged tile
+    // vs 278 us with three stages + per-thread loads (B = 512, N = 256)
+    sp.g_slots = 0;
+    sp.g_batched = d_acc_bstride != 0 ? 1 : 0;
+    CUtensorMap mgr = mq, mgr16 = mq;      // placeholders when the staged path is off (never dereferenced)
+    const bool g_ok = d_acc != nullptr && (d_acc_rstride & 3) == 0 && d_acc_rstride <= kTpad && (d_acc_bstride & 3) == 0 &&
+                      (reinterpret_cast<uintptr_t>(d_acc) & 15) == 0;
+    if (g_ok && stages_for(kGSlotBytes) >= 2) {
+      const int nb = sp.g_batched ? B : 1;
+      const int64_t bs = sp.g_batched ? d_acc_bstride : (int64_t)N * d_acc_rstride;
+      if ((rc = make_map_rows_f32(&mgr, d_acc, d_acc_rstride, N, nb, bs, 32, kM, CU_TENSOR_MAP_SWIZZLE_128B)) != GA_OK) return rc;
+      if ((rc = make_map_rows_f32(&mgr16, d_acc, d_acc_rstride, N, nb, bs, 16, kM, CU_TENSOR_MAP_SWIZZLE_64B)) != GA_OK) return rc;
+      sp.g_slots = 1;
     }
-    if (stream_mode != 0) {
-      BwdStreamParams sp;
-      sp.b = p;
-      const size_t kv = (size_t)2 * 2 * nblk * kKVBlockBytes, ring = (size_t)2 * kQBlockBytes;
-      auto stages_for = [&](size_t extra) {
-        for (int n = kMaxStages; n >= 2; --n)
-          if (1024 + kv + extra + n * ring <= 226 * 1024) return n;
-        return 0;
-      };
-      // TMA-staged map-gradient tile (40 KB) whenever the rows can be described to the TMA (16-byte aligned base and
-      // strides, at most 80 columns) and two ring stages remain: d = 160 runs 242 us with two stages + the staged tile
-      // vs 278 us with three stages + per-thread loads (B = 512, N = 256); GA_K2_GSTAGE=0 turns it off for A/B runs
-      static int g_mode = -2;
-      if (g_mode == -2) {
-        const char* eg = getenv("GA_K2_GSTAGE");
-        g_mode = eg == nullptr ? -1 : atoi(eg);
-      }
-      sp.g_slots = 0;
-      sp.g_batched = d_acc_bstride != 0 ? 1 : 0;
-      CUtensorMap mgr = mq, mgr16 = mq;      // placeholders when the staged path is off (never dereferenced)
-      const bool g_ok = d_acc != nullptr && (d_acc_rstride & 3) == 0 && d_acc_rstride <= kTpad && (d_acc_bstride & 3) == 0 &&
-                        (reinterpret_cast<uintptr_t>(d_acc) & 15) == 0;
-      if (g_ok && g_mode != 0 && stages_for(kGSlotBytes) >= 2) {
-        const int nb = sp.g_batched ? B : 1;
-        const int64_t bs = sp.g_batched ? d_acc_bstride : (int64_t)N * d_acc_rstride;
-        if ((rc = make_map_rows_f32(&mgr, d_acc, d_acc_rstride, N, nb, bs, 32, kM, CU_TENSOR_MAP_SWIZZLE_128B)) != GA_OK) return rc;
-        if ((rc = make_map_rows_f32(&mgr16, d_acc, d_acc_rstride, N, nb, bs, 16, kM, CU_TENSOR_MAP_SWIZZLE_64B)) != GA_OK) return rc;
-        sp.g_slots = 1;
-      }
-      const size_t g_bytes = sp.g_slots ? (size_t)kGSlotBytes : 0;
-      sp.ring_stages = stages_for(g_bytes);
-      if (sp.ring_stages >= 2) {
-        const size_t smem_s = 1024 + kv + sp.ring_stages * ring + g_bytes;
-        auto kern = sp.g_slots ? cross_attn_bwd_tc_stream_kernel<true> : cross_attn_bwd_tc_stream_kernel<false>;
-        cudaError_t es2 = ensure_smem(reinterpret_cast<const void*>(kern), sp.g_slots ? 7 : 5, smem_s);
-        if (es2 != cudaSuccess) return fail(GA_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(es2));
-        if (H > sm_count()) return fail(GA_ERR_UNSUPPORTED, "pipelined cross-attention backward: %d heads", H);
-        int teams_s = sm_count() / H;
-        if (teams_s > p.units) teams_s = p.units;
-        kern<<<teams_s * H, kPipeThreads, smem_s, st>>>(mq, mg, mk, mv, mgr, mgr16, sp);
-        return check_launch("cross_attn_bwd_tc_stream");
-      }
-    }
-    p.smem_stages = 1;
-    for (int n = kMaxStages; n >= 2; --n)
-      if (n * stage + 1024 <= 224 * 1024) { p.smem_stages = n; break; }
-    const size_t smem = p.smem_stages * stage + 1024;
-    if (smem > 224 * 1024) return fail(GA_ERR_UNSUPPORTED, "tcgen05 pipelined bwd: %zu B of shared memory", smem);
-    p.direct_store = (p.smem_stages == 2 || p.smem_stages == 3) ? 1 : 0;   // measured: staged wins again at 1 stage
-    CUtensorMap mdq;
-    if ((rc = make_map(&mdq, d_q, dtype, B, N, H, d, 32)) != GA_OK) return rc;   // one store per epilogue warp
-    cudaError_t e = ensure_smem(reinterpret_cast<const void*>(cross_attn_bwd_tc_pipe_kernel), 3, smem);
-    if (e != cudaSuccess) return fail(GA_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    const size_t g_bytes = sp.g_slots ? (size_t)kGSlotBytes : 0;
+    sp.ring_stages = stages_for(g_bytes);
+    // two stages fit for every head_dim <= 160: 1024 + 4 x 3 x 10240 + 2 x 32768 = 189 440 B
+    if (sp.ring_stages < 2) return fail(GA_ERR_UNSUPPORTED, "streaming tcgen05 cross-attention backward: head_dim %d", d);
+    const size_t smem_s = 1024 + kv + sp.ring_stages * ring + g_bytes;
+    auto kern = sp.g_slots ? cross_attn_bwd_tc_stream_kernel<true> : cross_attn_bwd_tc_stream_kernel<false>;
+    cudaError_t es2 = ensure_smem(reinterpret_cast<const void*>(kern), sp.g_slots ? 7 : 5, smem_s);
+    if (es2 != cudaSuccess) return fail(GA_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(es2));
     if (H > sm_count()) return fail(GA_ERR_UNSUPPORTED, "pipelined cross-attention backward: %d heads", H);
-    int teams = sm_count() / H;
-    if (teams > p.units) teams = p.units;
-    const int grid = teams * H;
-    cross_attn_bwd_tc_pipe_kernel<<<grid, kPipeThreads, smem, st>>>(mq, mg, mk, mv, mdq, p);
-    return check_launch("cross_attn_bwd_tc_pipe");
+    int teams_s = sm_count() / H;
+    if (teams_s > p.units) teams_s = p.units;
+    kern<<<teams_s * H, kPipeThreads, smem_s, st>>>(mq, mg, mk, mv, mgr, mgr16, sp);
+    return check_launch("cross_attn_bwd_tc_stream");
   }
   BwdParams p;
   p.d_q = d_q; p.lse = lse; p.d_acc = d_acc; p.d_acc_bstride = d_acc_bstride; p.d_acc_rstride = d_acc_rstride;

@@ -628,19 +628,17 @@ __device__ __forceinline__ void tail_bwd_rows(const float* a0, float* __restrict
 // non-zero only in the tracked tokens' columns, so a row of d_abar is the attn_text row of the same pixel scaled by one
 // per-pixel scalar (-k * sum_t a[col_t] dA_t), with n_tokens entries patched.  The kernel is therefore a shifted,
 // scaled row copy (75-float rows in, 80-float padded rows out) and is laid out for instruction count, which is what
-// bounded the previous version (ncu: issue slots 81 %, DRAM 36 %): one CTA owns `tile` pixels of one sample
-// (the whole 16x16 map, or 256 row-major pixels of a larger one plus a halo of one row + one pixel on each side for
-// the 3x3 filter adjoint); the per-token gradients dA_t are computed once per CTA, one thread per pixel; the streaming
-// phase gives every thread whole float4 chunks of the output (4 scalar loads, 4 multiplies, one 128-bit store).
-#ifndef GA_TAIL_BWD_MIN_CTAS
-#define GA_TAIL_BWD_MIN_CTAS 4
-#endif
+// bounded the previous version (ncu: issue slots 81 %, DRAM 36 %): one CTA owns `tile` row-major pixels of one sample
+// plus a halo of one row + one pixel on each side for the 3x3 filter adjoint; the per-token gradients dA_t are computed
+// once per CTA, one thread per pixel; the streaming phase gives every thread whole float4 chunks of the output (4 scalar
+// loads, 4 multiplies, one 128-bit store).
+constexpr int kTailBwdMinCtas = 4;    // resident CTAs per SM the register allocation must allow
 // (round 2, second pass) The tile's attn_text rows -- tile x 75 contiguous floats -- are fetched by ONE bulk copy
 // (cp.async.bulk global -> shared, mbarrier complete_tx) issued before anything else, so the stream is in flight while
 // phases 1-2 chase their small dependent loads; phase 2 and the row phase then read shared memory.  Before, a CTA's
 // global row loads only started after two __syncthreads (ncu: 40 % of the stall samples sat in phases 1-2 with the
 // memory pipe idle).
-__global__ void __launch_bounds__(kThreads, GA_TAIL_BWD_MIN_CTAS)
+__global__ void __launch_bounds__(kThreads, kTailBwdMinCtas)
 tail_bwd_sparse_kernel(ga_tail_params_t p, TokArgs toks, const uint8_t* __restrict__ masks,
                        const float* __restrict__ weights, const float* __restrict__ attn_text,
                        const float* __restrict__ smoothed, const float* __restrict__ stats,
@@ -995,14 +993,8 @@ extern "C" int ga_guidance_tail_bwd(const ga_tail_params_t* params_host, const g
   if ((d_abar_row_stride & 3) == 0) GA_CHECK_ALIGN(d_abar, 16, "d_abar");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (g_attn_text == nullptr && (d_abar_row_stride & 3) == 0) {
-    // the pipeline's case: sparse map gradient.  Large launches give a CTA 256 pixels (a whole 16x16 map: no halo at
-    // all); small ones 64, so that a single evaluation still spreads over a few SMs.
-    static int tile_env = -1;
-    if (tile_env < 0) {
-      const char* e = getenv("GA_TAIL_BWD_TILE");
-      tile_env = e != nullptr ? atoi(e) : 0;
-    }
-    const int tile = tile_env > 0 ? (tile_env & ~3) : 128;
+    // the pipeline's case: sparse map gradient.  A CTA owns 128 pixels (half of a 16x16 map) and their halo.
+    const int tile = 128;
     const int nt = p.n_tokens > 0 ? p.n_tokens : 1;
     const int tp = p.last - p.first;
     const size_t smem = ((size_t)tile * tp + (size_t)nt * (3 * tile + 2 * (p.res + 1)) + tile) * sizeof(float);

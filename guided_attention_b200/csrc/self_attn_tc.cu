@@ -4,19 +4,19 @@
 // SURVEY.md section 8 row f4.  These layers are off the guidance path (their maps are never read) but on the autograd
 // path, so the backward is provided too.
 //
-// Forward, one CTA = 128 query rows of one (batch, head), two passes over the keys in blocks of BK (128 or 64):
-//   pass 1   S_j = Q K_j^T -> running row maximum                      (no exponentials)
-//   pass 2   S_j again -> P_j = exp(scale (S_j - max)) (un-normalised, 16-bit, back into TMEM) -> O += P_j V_j
-//            with the row sum accumulated on the side; O is divided by the sum once, in the epilogue.
-// With the final maximum known before the first exponential, O never has to be rescaled (no correction pass over the
-// TMEM accumulator); the price is a second QK^T GEMM per block, which is free here -- the kernel is bound by the
-// exponentials and the TMEM <-> register traffic, not by the tensor pipe or HBM (K and V blocks come from L2).
+// Forward, one CTA = 128 query rows of one (batch, head), ONE pass over the keys in blocks of BK (128 or 64) with an
+// online softmax: per block S_j = Q K_j^T, P_j = exp(scale (S_j - running max)) (un-normalised, 16-bit, back into
+// TMEM), O += P_j V_j.  The two compute groups own alternate key blocks, each with its own output accumulator and
+// running max / sum; the epilogue merges the two partial results and divides by the row sum once.
 //
-//   warp 0      TMA producer   Q tile once, then a ring of K (pass 1) / K+V (pass 2) blocks
-//   warp 1      MMA issuer     MMA1 into S buffer g = item & 1; MMA2(item-2) is issued before MMA1(item), which is what
-//                              orders "P consumed" before "S overwritten" (tcgen05.mma retires in issue order)
-//   warps 4-7   compute group 0 (S buffer 0), warps 8-11 compute group 1 (S buffer 1): thread = query row = TMEM lane;
-//               the two groups own alternate key blocks and merge their row maxima / sums through shared memory.
+//   warp 0      TMA producer   Q tile once, then a ring of K+V blocks
+//   warp 1      MMA issuer 1   S(j) = Q K_j^T into score buffer j % 3
+//   warp 2      MMA issuer 2   O_(j & 1) += P(j) V_j; its commit frees the K/V stage and the score buffer
+//   warps 4-7   compute group 0 (even key blocks), warps 8-11 compute group 1 (odd key blocks): thread = query row =
+//               TMEM lane.
+// Three score buffers for two groups: the scores of a group's next block are computed while it works on the current
+// one, and the two issuers are ordered by completion (P_FREE), not by sharing one instruction stream -- with a single
+// issuer warp and two buffers every group waited a full issue -> tensor pipe -> commit round trip per block.
 #include "tc_common.cuh"
 
 namespace ga {
@@ -51,280 +51,21 @@ struct RingPos {
   }
 };
 
-// Forward roles:
-//   warp 0      TMA producer   Q tile once, then a ring of K (pass 1) / K+V (pass 2) blocks
-//   warp 1      MMA issuer 1   S(it) = Q K_j^T into score buffer it % 3
-//   warp 2      MMA issuer 2   O += P(it) V_j for the pass-2 items; its commit also frees the score buffer
-//   warps 4-7   compute group 0, warps 8-11 compute group 1: thread = query row = TMEM lane; the groups own alternate
-//               key blocks and merge their row maxima / sums through shared memory.
-// Three score buffers for two groups: the scores of a group's next block are computed while it works on the current
-// one, and the two issuers are ordered by completion (P_FREE), not by sharing one instruction stream -- with a single
-// issuer warp and two buffers every group waited a full issue -> tensor pipe -> commit round trip per block.
-__global__ void __launch_bounds__(kThreads, 1)
-self_attn_fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
-                     const __grid_constant__ CUtensorMap map_v, const FwdParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  // q_full, o_ready, kv_full[4], kv_free[4], s_ready[3], p_ready[3], p_free[3]
-  __shared__ __align__(8) uint64_t bars[19];
-  __shared__ uint32_t tmem_base_slot;
-  __shared__ float xchg[2][kM];          // row maxima / sums of the two compute groups
-
-  const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
-  const int tile = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
-  const int row0 = tile * kM;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t kv_block_bytes = (uint32_t)p.bk * 128u;                  // one 64-channel block of K or V
-  const uint32_t k_bytes = (uint32_t)p.nblk * kv_block_bytes;
-  const uint32_t stage_bytes = 2u * k_bytes;
-  const uint32_t sQ = base;
-  const uint32_t sKV = sQ + (uint32_t)p.nblk * kQBlockBytes;
-  auto Q_FULL = [&]() { return smem_u32(&bars[0]); };
-  auto O_READY = [&]() { return smem_u32(&bars[1]); };
-  auto KV_FULL = [&](int s) { return smem_u32(&bars[2 + s]); };
-  auto KV_FREE = [&](int s) { return smem_u32(&bars[6 + s]); };
-  auto S_READY = [&](int i) { return smem_u32(&bars[10 + i]); };
-  auto P_READY = [&](int i) { return smem_u32(&bars[13 + i]); };
-  auto P_FREE = [&](int i) { return smem_u32(&bars[16 + i]); };
-  const uint32_t colO = (uint32_t)(kSBuf * p.bk);
-
-  if (tid == 0) {
-    prefetch_tmap(&map_q); prefetch_tmap(&map_k); prefetch_tmap(&map_v);
-    mbar_init(Q_FULL(), 1);
-    mbar_init(O_READY(), 1);
-    for (int s = 0; s < kMaxStages; ++s) { mbar_init(KV_FULL(s), 1); mbar_init(KV_FREE(s), 1); }
-    for (int i = 0; i < kSBuf; ++i) {
-      mbar_init(S_READY(i), 1);
-      mbar_init(P_READY(i), kGroupThreads);
-      mbar_init(P_FREE(i), 1);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 0) tmem_alloc(smem_u32(&tmem_base_slot), 512u);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = uniform_u32(tmem_base_slot);
-  const int nb = p.nb, n_items = 2 * nb, NS = p.stages;
-  const int ksteps = (p.d + 15) >> 4;
-  const int fmt = p.bf16 ? 1 : 0;
-
-  if (warp < 4) {
-    reg_dealloc<40>();
-    if (warp == 0) {
-      // ------------------------------------------------------------------------------------------- producer
-      if (elect_one()) {
-        mbar_expect_tx(Q_FULL(), (uint32_t)p.nblk * kQBlockBytes);
-        for (int blk = 0; blk < p.nblk; ++blk)
-          tma_load_4d(sQ + blk * kQBlockBytes, &map_q, Q_FULL(), blk * kBlockCols, h, row0, b);
-      }
-      RingPos st = {0, 0};
-      int j = 0;
-      for (int it = 0; it < n_items; ++it) {
-        const bool with_v = it >= nb;
-        if (it >= NS) mbar_wait(KV_FREE(st.idx), st.par ^ 1u);
-        if (elect_one()) {
-          const uint32_t sK = sKV + st.idx * stage_bytes, sV = sK + k_bytes;
-          mbar_expect_tx(KV_FULL(st.idx), with_v ? stage_bytes : k_bytes);
-          for (int blk = 0; blk < p.nblk; ++blk) {
-            tma_load_4d(sK + blk * kv_block_bytes, &map_k, KV_FULL(st.idx), blk * kBlockCols, h, j * p.bk, b);
-            if (with_v) tma_load_4d(sV + blk * kv_block_bytes, &map_v, KV_FULL(st.idx), blk * kBlockCols, h, j * p.bk, b);
-          }
-        }
-        __syncwarp();
-        if (++j == nb) j = 0;
-        st.advance(NS);
-      }
-    } else if (warp == 1) {
-      // ----------------------------------------------------------------------------- MMA issuer 1: S = Q K^T
-      const uint32_t idesc_qk = make_idesc(fmt, 0, p.bk, kM);
-      const uint64_t dQ0 = smem_desc_sw128(sQ, 16, 1024);
-      const uint64_t dK0 = smem_desc_sw128(sKV, 16, 1024);                          // stage 0, K-major
-      mbar_wait(Q_FULL(), 0);
-      RingPos st = {0, 0}, sb = {0, 0};
-      uint32_t pfree_par[kSBuf] = {0, 0, 0};       // parity of the next P_FREE completion to consume, per buffer
-      for (int it = 0; it < n_items; ++it) {
-        if (it >= kSBuf) {
-          // the buffer's previous item (it - 3): its rows have been read (pass 1) / its P written (pass 2) ...
-          mbar_wait(P_READY(sb.idx), sb.par ^ 1u);
-          if (it - kSBuf >= nb) {                  // ... and consumed by its PV GEMM
-#pragma unroll
-            for (int i = 0; i < kSBuf; ++i)
-              if (i == sb.idx) { mbar_wait(P_FREE(i), pfree_par[i]); pfree_par[i] ^= 1u; }
-          }
-        }
-        mbar_wait(KV_FULL(st.idx), st.par);
-        tc_fence_after();
-        if (elect_one()) {
-          issue_kmajor_gemm(tmem + (uint32_t)(sb.idx * p.bk), dQ0, kQBlockBytes, desc_advance(dK0, st.idx * stage_bytes),
-                            kv_block_bytes, ksteps, idesc_qk);
-          tc_commit(S_READY(sb.idx));
-          if (it < nb) tc_commit(KV_FREE(st.idx));     // pass 1: the block is only needed by this GEMM
-        }
-        __syncwarp();
-        st.advance(NS);
-        sb.advance(kSBuf);
-      }
-    } else if (warp == 2) {
-      // ----------------------------------------------------------------------------- MMA issuer 2: O += P V
-      const uint32_t idesc_pv = make_idesc(fmt, 1, p.npv, kM);
-      const uint64_t dV0 = smem_desc_sw128(sKV + k_bytes, kv_block_bytes, 1024);    // stage 0, MN-major
-      const int pv_steps = p.bk / 16;
-      // Every item's P_READY is waited for in order, pass-1 items included: a parity wait can only tell "this use" from
-      // "the previous one", so jumping straight to the first pass-2 use of a buffer would sail through a phase that has
-      // not even started.
-      RingPos st = {0, 0}, sb = {0, 0};
-      for (int it = 0; it < n_items; ++it) {
-        mbar_wait(P_READY(sb.idx), sb.par);
-        tc_fence_after();
-        if (it >= nb && elect_one()) {
-          issue_tmem_gemm(tmem + colO, tmem + (uint32_t)(sb.idx * p.bk), desc_advance(dV0, st.idx * stage_bytes), pv_steps,
-                          idesc_pv, it > nb);
-          tc_commit(KV_FREE(st.idx));
-          tc_commit(P_FREE(sb.idx));
-        }
-        __syncwarp();
-        st.advance(NS);
-        sb.advance(kSBuf);
-      }
-      if (elect_one()) tc_commit(O_READY());
-      __syncwarp();
-    }
-  } else {
-    reg_alloc<232>();
-    // --------------------------------------------------------------------------------------- compute groups
-    const int g = (warp - 4) >> 2;
-    const int r = ((warp & 3) << 5) + lane;
-    const int row = row0 + r;
-    const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-    const float sc = p.scale * 1.4426950408889634f;
-    const bool bf16 = p.bf16 != 0;
-    const int halves = p.bk / 64;                    // S is processed 64 key columns at a time
-
-    // ---- pass 1: running maximum over this group's key blocks (four independent chains)
-    float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-    for (int it = g; it < nb; it += 2) {
-      const int buf = it % kSBuf;
-      const uint32_t colS = (uint32_t)(buf * p.bk);
-      mbar_wait(S_READY(buf), (uint32_t)(it / kSBuf) & 1u);
-      tc_fence_after();
-      const int key0 = it * p.bk;
-      const bool ragged = key0 + p.bk > p.N;
-      for (int hf = 0; hf < halves; ++hf) {
-        float s[64];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) tmem_ld16(lane_base + colS + hf * 64 + c * 16, s + c * 16);
-        tmem_ld_wait();
-        if (!ragged) {
-#pragma unroll
-          for (int j = 0; j < 64; ++j) m4[j & 3] = fmaxf(m4[j & 3], s[j]);
-        } else {
-#pragma unroll
-          for (int j = 0; j < 64; ++j)
-            if (key0 + hf * 64 + j < p.N) m4[j & 3] = fmaxf(m4[j & 3], s[j]);
-        }
-      }
-      tc_fence_before();
-      mbar_arrive(P_READY(buf));
-    }
-    float m = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
-    xchg[g][r] = m;
-    named_bar_sync(1, 2 * kGroupThreads);
-    m = fmaxf(xchg[0][r], xchg[1][r]);
-    named_bar_sync(2, 2 * kGroupThreads);            // both groups have read the maxima before the sums reuse xchg
-    const float mo = m * sc;
-
-    // ---- pass 2: P = exp(scale (S - max)) -> TMEM, row sum on the side
-    float l4[4] = {0.f, 0.f, 0.f, 0.f};
-    for (int it = nb + ((nb & 1) ^ g); it < n_items; it += 2) {      // items of this group: it & 1 == g
-      const int buf = it % kSBuf;
-      const uint32_t colS = (uint32_t)(buf * p.bk);
-      mbar_wait(S_READY(buf), (uint32_t)(it / kSBuf) & 1u);
-      tc_fence_after();
-      const int key0 = (it - nb) * p.bk;
-      const bool ragged = key0 + p.bk > p.N;
-      for (int hf = 0; hf < halves; ++hf) {
-        float s[64];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) tmem_ld16(lane_base + colS + hf * 64 + c * 16, s + c * 16);
-        tmem_ld_wait();
-        if (!ragged) {
-#pragma unroll
-          for (int j = 0; j < 64; ++j) { s[j] = ex2_approx(fmaf(s[j], sc, -mo)); l4[j & 3] += s[j]; }
-        } else {
-#pragma unroll
-          for (int j = 0; j < 64; ++j) {
-            s[j] = (key0 + hf * 64 + j < p.N) ? ex2_approx(fmaf(s[j], sc, -mo)) : 0.f;
-            l4[j & 3] += s[j];
-          }
-        }
-        // the second half of S must be in registers before P overwrites the head of the buffer: with bk = 128 the P
-        // columns of half 0 (0..31) do not overlap the S columns of half 1 (64..127), and half 1's P goes to 32..63
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          uint32_t packed[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) packed[i] = pack16(s[c * 16 + 2 * i], s[c * 16 + 2 * i + 1], bf16);
-          tmem_st8(lane_base + colS + hf * 32 + c * 8, packed);
-        }
-      }
-      tmem_st_wait();
-      tc_fence_before();
-      mbar_arrive(P_READY(buf));
-    }
-    float l = (l4[0] + l4[1]) + (l4[2] + l4[3]);
-    xchg[g][r] = l;
-    named_bar_sync(3, 2 * kGroupThreads);
-    l = xchg[0][r] + xchg[1][r];
-    const float inv = 1.f / l;
-    if (g == 0 && row < p.N) p.lse[((int64_t)b * p.H + h) * p.N + row] = m * p.scale + logf(l);
-
-    // ---- epilogue: the two groups take alternate 16-column chunks of O
-    mbar_wait(O_READY(), 0);
-    tc_fence_after();
-    uint8_t* orow = reinterpret_cast<uint8_t*>(p.o) + (((int64_t)b * p.N + row) * p.H + h) * (int64_t)p.d * 2;
-    for (int cc = g; cc < p.npv / 16; cc += 2) {
-      float ov[16];
-      tmem_ld16(lane_base + colO + cc * 16, ov);
-      tmem_ld_wait();
-      if (row < p.N) {
-        uint32_t w[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) w[i] = pack16(ov[2 * i] * inv, ov[2 * i + 1] * inv, bf16);
-        const int col = cc * 16;
-        if (col < p.d) *reinterpret_cast<uint4*>(orow + col * 2) = make_uint4(w[0], w[1], w[2], w[3]);
-        if (col + 8 < p.d) *reinterpret_cast<uint4*>(orow + col * 2 + 16) = make_uint4(w[4], w[5], w[6], w[7]);
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem, 512u);
-}
-
-// ================================================================================ forward, single pass (default)
-// One pass over the keys with an online softmax, so QK^T is issued once (2 GEMMs per key block instead of 3) and the
-// scores cross TMEM -> registers once.  Each compute group keeps its OWN output accumulator in TMEM (O_0 for the even
-// key blocks, O_1 for the odd ones) together with its own running row maximum and row sum, so the groups never have
-// to agree on a maximum while the blocks stream; the epilogue merges the two partial results
+// ============================================================================================ forward
+// QK^T is issued once per key block and the scores cross TMEM -> registers once.  Each compute group keeps its OWN
+// output accumulator in TMEM (O_0 for the even key blocks, O_1 for the odd ones) together with its own running row
+// maximum and row sum, so the groups never have to agree on a maximum while the blocks stream; the epilogue merges the
+// two partial results
 //     m = max(m_0, m_1),  l = l_0 2^(m_0 - m) + l_1 2^(m_1 - m),  O = (O_0 2^(m_0 - m) + O_1 2^(m_1 - m)) / l.
 // The running maximum is LAZY: a group keeps exponentiating against a stale maximum as long as the block maximum
 // exceeds it by less than 2^kLazyBits (P <= 256: harmless for the 16-bit P operand and the fp32 sums), and only when a
 // row jumps further does its warp rescale its O accumulator in TMEM (tcgen05.ld -> multiply -> tcgen05.st, after the
 // group's previous PV GEMM has completed).  After the first block of a group that is rare, so the common path of a
-// block is: tcgen05.ld S -> max -> exp2 -> sum -> pack -> tcgen05.st P -> arrive.
+// block is: tcgen05.ld S -> max -> exp2 -> sum -> pack -> tcgen05.st P -> arrive.  Every exponential runs on the SFU:
+// handing some of them to the FMA pipe as a polynomial measured slower (profiles/r02_microbench_self_attn_poly_ab.txt).
 //
 //   TMEM:  3 score buffers of `bk` columns | O_0 (npv) | O_1 (npv)      (d = 160: 192 + 320 = 512 columns)
-//   roles as in the two-pass kernel below: warp 0 TMA producer, warp 1 issuer of S = Q K_j^T, warp 2 issuer of
-//   O_g += P_j V_j (its commit frees the K/V stage and the score buffer), warps 4-7 / 8-11 compute groups.
 constexpr float kLazyBits = 8.f;
-// Every kPolyEvery-th exponential can be handed to the FMA pipe (tc::ex2_poly3, the FA-4 trick).  Measured on B200 at
-// N = 4096, d = 40 (profiles/r02_microbench_self_attn_poly_ab.txt): 58.0 us with every exponential on the SFU, 59.3-59.8 us
-// with every 4th / 6th / 8th on the FMA pipe -- the kernel is not SFU-bound enough (XU 64 %, issue slots 42 %) for the
-// nine extra issue slots per polynomial to pay, so the default is off.
-#ifndef GA_SA_POLY_EVERY
-#define GA_SA_POLY_EVERY 0
-#endif
-constexpr int kPolyEvery = GA_SA_POLY_EVERY;
 
 template <int BK>
 __global__ void __launch_bounds__(kThreads, 1)
@@ -498,8 +239,7 @@ self_attn_fwd1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
       const float mo = m_used * sc;
 #pragma unroll
       for (int j = 0; j < BK; ++j) {
-        const float x = fmaf(s[j], sc, -mo);
-        s[j] = (kPolyEvery > 0 && (j % (kPolyEvery > 0 ? kPolyEvery : 1)) == kPolyEvery - 1) ? ex2_poly3(x) : ex2_approx(x);
+        s[j] = ex2_approx(fmaf(s[j], sc, -mo));
         l4[j & 3] += s[j];
       }
       // P (packed 16-bit, BK / 2 columns) over the head of the score buffer: every score is in registers by now
@@ -575,6 +315,9 @@ int fwd(const void* q, const void* k, const void* v, void* o, float* lse, int B,
   for (int n = kMaxStages; n >= 2; --n)
     if (1024 + q_bytes + n * stage <= 226 * 1024) { p.stages = n; break; }
   if (p.stages == 0) return fail(GA_ERR_UNSUPPORTED, "self-attention: head_dim %d does not fit shared memory", d);
+  // two output accumulators behind the three score buffers: 3 bk + 2 npv <= 512 TMEM columns (every head_dim <= 160)
+  if (kSBuf * p.bk + 2 * p.npv > 512)
+    return fail(GA_ERR_UNSUPPORTED, "self-attention: head_dim %d does not fit tensor memory", d);
   const size_t smem = 1024 + q_bytes + p.stages * stage;
   CUtensorMap mq, mk, mv;
   int rc;
@@ -582,26 +325,13 @@ int fwd(const void* q, const void* k, const void* v, void* o, float* lse, int B,
   if ((rc = make_map(&mk, k, dtype, B, N, H, d, p.bk)) != GA_OK) return rc;
   if ((rc = make_map(&mv, v, dtype, B, N, H, d, p.bk)) != GA_OK) return rc;
   dim3 grid((N + kM - 1) / kM, H, B);
-  // GA_SA_TWO_PASS=1 selects the round-1 two-pass kernel (A/B measurements); the single-pass kernel needs two output
-  // accumulators behind the three score buffers: 3 bk + 2 npv <= 512 TMEM columns (true for every head_dim <= 160)
-  static int two_pass = -1;
-  if (two_pass < 0) {
-    const char* e2 = getenv("GA_SA_TWO_PASS");
-    two_pass = (e2 != nullptr && e2[0] == '1') ? 1 : 0;
-  }
-  if (two_pass == 0 && kSBuf * p.bk + 2 * p.npv <= 512) {
-    const void* kern = p.bk == 128 ? reinterpret_cast<const void*>(self_attn_fwd1_kernel<128>)
-                                   : reinterpret_cast<const void*>(self_attn_fwd1_kernel<64>);
-    cudaError_t e1 = ensure_smem(kern, p.bk == 128 ? 4 : 5, smem);
-    if (e1 != cudaSuccess) return fail(GA_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e1));
-    if (p.bk == 128) self_attn_fwd1_kernel<128><<<grid, kThreads, smem, st>>>(mq, mk, mv, p);
-    else self_attn_fwd1_kernel<64><<<grid, kThreads, smem, st>>>(mq, mk, mv, p);
-    return check_launch("self_attn_fwd1");
-  }
-  cudaError_t e = ensure_smem(reinterpret_cast<const void*>(self_attn_fwd_kernel), 0, smem);
+  const void* kern = p.bk == 128 ? reinterpret_cast<const void*>(self_attn_fwd1_kernel<128>)
+                                 : reinterpret_cast<const void*>(self_attn_fwd1_kernel<64>);
+  cudaError_t e = ensure_smem(kern, p.bk == 128 ? 4 : 5, smem);
   if (e != cudaSuccess) return fail(GA_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-  self_attn_fwd_kernel<<<grid, kThreads, smem, st>>>(mq, mk, mv, p);
-  return check_launch("self_attn_fwd");
+  if (p.bk == 128) self_attn_fwd1_kernel<128><<<grid, kThreads, smem, st>>>(mq, mk, mv, p);
+  else self_attn_fwd1_kernel<64><<<grid, kThreads, smem, st>>>(mq, mk, mv, p);
+  return check_launch("self_attn_fwd1");
 }
 
 

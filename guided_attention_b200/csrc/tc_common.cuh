@@ -149,20 +149,6 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
-// 2^x on the FMA pipe (no MUFU): Cody-Waite split x = n + f, f in [-0.5, 0.5], degree-3 minimax polynomial for 2^f
-// (max relative error 7.5e-5 -- below the 2^-11 rounding of the 16-bit P operand it feeds), n added to the exponent
-// bits.  9 FMA/ALU-pipe instructions, i.e. the same issue cost as one MUFU.EX2 at the SM's 16/clk SFU rate; an A/B
-// option of the self-attention forward (GA_SA_POLY_EVERY, off by default: measured slower, see self_attn_tc.cu).  x <= ~8 here; x below -126 (masked keys: -inf) gives 2^-126 ~ 0.
-__device__ __forceinline__ float ex2_poly3(float x) {
-  x = fmaxf(x, -126.f);
-  const float t = x + 12582912.f;                    // 1.5 * 2^23: the low mantissa bits of t now hold round(x)
-  const float f = x - (t - 12582912.f);
-  float pl = fmaf(0.055171169340610504f, f, 0.24261002242565155f);
-  pl = fmaf(pl, f, 0.6932609677314758f);
-  pl = fmaf(pl, f, 0.9999281167984009f);
-  return __int_as_float(__float_as_int(pl) + (__float_as_int(t) << 23));
-}
-
 // ---- warp-uniform role helpers ----------------------------------------------------------------------------------
 // The TMA-producer and MMA-issuer roles run as WHOLE warps in warp-uniform control flow and pick one lane with
 // elect.sync for the asynchronous instructions.  A role entered through a divergent `lane == 0` branch makes the
@@ -215,11 +201,6 @@ __device__ __forceinline__ void issue_tmem_gemm(uint32_t d_tmem, uint32_t a_tmem
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2, int c3) {
   asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
                ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
-// 1-D bulk copy shared -> global (16-byte aligned addresses, size a multiple of 16), tracked by the thread's bulk group
-__device__ __forceinline__ void bulk_store_1d(void* dst, uint32_t src_smem, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src_smem), "r"(bytes)
                : "memory");
 }
 __device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
@@ -278,9 +259,6 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 }
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-__device__ __forceinline__ void named_bar_arrive(int id, int nthreads) {
-  asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 template <int kRegs> __device__ __forceinline__ void reg_dealloc() {
   asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegs));

@@ -463,16 +463,6 @@ int64_t ws_bytes(int n, int hw, int c, int groups) {
   return (int64_t)n * p.P * groups * 2 * (int64_t)sizeof(float);
 }
 
-// GA_GN_PDL=0 launches the second kernel of a pair as an ordinary stream-ordered launch (A/B measurements).
-static bool use_pdl() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GA_GN_PDL");
-    v = (e != nullptr && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
-
 template <typename K>
 static void launch_second(K kernel, const dim3& grid, const Params& p, cudaStream_t st) {
   cudaLaunchConfig_t cfg = {};
@@ -484,7 +474,7 @@ static void launch_second(K kernel, const dim3& grid, const Params& p, cudaStrea
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = use_pdl() ? 1 : 0;
+  cfg.numAttrs = 1;
   cudaLaunchKernelEx(&cfg, kernel, p);
 }
 

@@ -309,11 +309,9 @@ def cross_attention(q, k, v, heads: int, scale: float, want_acc: bool = False, i
 
 
 def self_attn_flops(B, H, N, d, direction="fwd"):
-    """Tensor-core FLOPs one launch pair issues: the single-pass forward runs the algorithm's 2 GEMMs (the round-1
-    two-pass kernel, GA_SA_TWO_PASS=1, issues 3); the backward runs 7 for the algorithm's 5."""
-    import os
-    fwd = 3 if os.environ.get("GA_SA_TWO_PASS", "0") == "1" else 2
-    return (fwd if direction == "fwd" else 7) * 2 * B * H * N * N * d
+    """Tensor-core FLOPs one launch pair issues: the forward runs the algorithm's 2 GEMMs; the backward runs 7 for the
+    algorithm's 5."""
+    return (2 if direction == "fwd" else 7) * 2 * B * H * N * N * d
 
 
 def self_attention_forward(q, k, v, heads: int, scale: float):
